@@ -64,7 +64,12 @@ def parse_args():
     ap.add_argument("--word-timestamps", action="store_true", help="BASELINE config 4: K14 word alignment on every chunk (e2e only)")
     ap.add_argument("--no-streaming", action="store_true", help="skip the staggered-arrival latency phase (RoundScheduler, step-level admission)")
     ap.add_argument("--stream-load", type=float, default=0.6, help="offered load of the streaming phase as a fraction of the batch throughput")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last step of each timed path "
+                    "returned as DIR/<name>.npy (float64; rank 0's streams for the resident path)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def tokens_for(seconds: float) -> int:
@@ -232,10 +237,13 @@ def main():
             dist.barrier()
         torch.cuda.synchronize()
 
+    last = {}   # what the latest step of each timed path returned (--dump-outputs)
+
     def e2e_step():
         t0 = time.perf_counter()
         out = dist_tr.transcribe_batch(waves, all_kws)      # whole batch in, whole batch out on every rank
         n_ids = sum(len(s.tokens) for segs, _ in out for s in (segs or []))
+        last["e2e"] = out
         return time.perf_counter() - t0, n_ids
 
     # ---- resident-input step: PCM / features already in HBM, device-timed
@@ -251,7 +259,7 @@ def main():
         rc = eng.lib.wl_encode_resident(eng.ctx, len(slots), _lib.ptr(slots, C.c_int32))
         _lib.check(eng.lib, eng.ctx, rc, "wl_encode_resident")
         ms += eng.last_device_ms(1)
-        eng.generate(feats_cache["enc"], feats_cache["prompts"], **feats_cache["gen_kw"])
+        last["resident"] = eng.generate(feats_cache["enc"], feats_cache["prompts"], **feats_cache["gen_kw"])
         ms += eng.last_device_ms(2)
         return ms / 1000.0
 
@@ -303,6 +311,8 @@ def main():
     barrier()
     t_e2e = time.perf_counter() - t0
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, eng, feats_cache["enc"], last["resident"], last["e2e"])
 
     loop_ms, loop_steps = eng.last_device_ms(2), getattr(eng, "last_steps", None)   # the last e2e step's decode loop
     # ---- streaming phase: staggered arrivals through the product scheduler (N=1 rank-local; reported, not the headline)
@@ -367,6 +377,34 @@ def main():
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
+
+
+def dump_outputs(out_dir: str, eng, enc, resident, e2e):
+    """The last timed step's results as float64 arrays, padded with -1 where lengths differ.
+
+    resident_*: what ``generate`` returned for this rank's streams (best hypothesis), and the encoder output it decoded
+    from -- 64 frames per stream drawn with a fixed seed, all channels.  e2e_*: what ``transcribe_batch`` returned for
+    every stream: segment tokens, and one row per segment (stream, start, end, avg_logprob, no_speech_prob,
+    compression_ratio)."""
+    os.makedirs(out_dir, exist_ok=True)
+
+    def padded(rows):
+        a = np.full((len(rows), max([len(r) for r in rows] + [1])), -1.0)
+        for i, r in enumerate(rows):
+            a[i, :len(r)] = r
+        return a
+    frames = np.sort(np.random.default_rng(0).choice(1500, 64, replace=False))
+    arrays = {
+        "resident_tokens": padded([r.sequences_ids[0] for r in resident]),
+        "resident_scores": np.array([r.scores[0] for r in resident], dtype=np.float64),
+        "resident_no_speech_prob": np.array([r.no_speech_prob for r in resident], dtype=np.float64),
+        "resident_encoder_output_sample": np.stack([eng._encoder_output(s)[frames] for s in enc.slots]).astype(np.float64),
+        "e2e_tokens": padded([[t for s in (segs or []) for t in s.tokens] for segs, _ in e2e]),
+        "e2e_segments": np.array([[i, s.start, s.end, s.avg_logprob, s.no_speech_prob, s.compression_ratio]
+                                  for i, (segs, _) in enumerate(e2e) for s in (segs or [])], dtype=np.float64).reshape(-1, 6),
+    }
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def streaming_latency(model, waves, kws, durs, batch_step_s: float, load: float, cycles: int = 3, step_tokens: int = 16):

@@ -6,14 +6,12 @@ import re
 import subprocess
 import sys
 import threading
-import time
 
 import numpy as np
 import pytest
 import torch
 
 ROOT = os.path.abspath(os.path.join(os.path.dirname(__file__), ".."))
-REF = "/root/reference"
 
 
 def test_c_abi_exports_every_declared_symbol():
@@ -209,56 +207,51 @@ def test_step_scheduler_joins_the_running_decode_loop():
         assert [(s.start, s.end) for s in r.result] == [(s.start, s.end) for s in segs]
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present")
 def test_backend_plugin_streams_segments_through_reference_base():
-    """ServeClientB200 subclasses the reference's ServeClientBase; frames go in through add_frames and
-    segment JSON comes out of the reference's own send path."""
-    sys.path.insert(0, REF)
-    try:
-        from whisperlive_b200 import synth
-        from whisperlive_b200.backend import ServeClientB200
-        from whisper_live.backend.base import ServeClientBase
-    finally:
-        sys.path.remove(REF)
-    assert issubclass(ServeClientB200, ServeClientBase)
-    torch.set_num_threads(8)
+    """ServeClientB200 subclasses the reference's ServeClientBase; frames go in through the base's loop and segment JSON
+    comes out of the base's send path.  tests/golden/record_plugin_base.py ran the plugin on the reference's own base and
+    recorded every call across that boundary; here a stand-in base replays the record: its loop hands the plugin the
+    same audio chunk and duration, and every call the plugin makes into the base (update_segments, prepare_segments,
+    send_transcription_to_client) must come in the recorded order with the recorded arguments, and gets the reference
+    base's answer back.  The plugin's own websocket messages and its transcription result must match too."""
+    import importlib
 
-    class WS:
-        def __init__(self):
-            self.sent, self.closed = [], False
-
-        def send(self, msg):
-            self.sent.append(json.loads(msg))
-
-        def close(self):
-            self.closed = True
-    model = _oracle_model()
-    # keep the CPU oracle cheap: the plugin's requests carry the reference defaults (beam 5, six-rung temperature ladder,
-    # up to 224 new tokens), which is tens of seconds per chunk on the oracle and trips base.py's 30 s request timeout
+    from tests.golden import record_plugin_base as R
+    import whisperlive_b200.backend as backend
     from whisperlive_b200.scheduler import BatchRequest
+    torch.set_num_threads(8)
+    rec = json.load(open(os.path.join(ROOT, "tests", "golden", "plugin_base_calls.json")))
+    stand_in = R.replay_module(rec)
+    names = ("whisper_live", "whisper_live.backend", "whisper_live.backend.base")
+    saved = {n: sys.modules.get(n) for n in names}
+    sys.modules.update(zip(names, (type(sys)("whisper_live"), type(sys)("whisper_live.backend"), stand_in)))
     orig_kwargs = BatchRequest.kwargs
-    BatchRequest.kwargs = lambda self: dict(orig_kwargs(self), temperature=[0.0], beam_size=2, log_prob_threshold=None,
-                                            max_new_tokens=24)
-    ServeClientB200.MODEL_FACTORY = lambda name: model
-    ws = WS()
+    BatchRequest.kwargs = lambda self: dict(orig_kwargs(self), **R.CHEAP)
     try:
-        client = ServeClientB200(ws, client_uid="u1", model="micro.en", use_vad=False, no_speech_thresh=1.1)
-        assert ws.sent[0] == {"uid": "u1", "message": "SERVER_READY", "backend": "faster_whisper"}
+        ServeClientB200 = importlib.reload(backend).ServeClientB200
+        assert issubclass(ServeClientB200, stand_in.ServeClientBase)
+        model = _oracle_model()
+        ServeClientB200.MODEL_FACTORY = lambda name: model
+        ws = R.WS()
+        client = ServeClientB200(ws, **R.CLIENT)
         assert client.language == "en"
-        client.add_frames(synth.speech_like(3.0, seed=1))
-        deadline = time.time() + 60
-        while time.time() < deadline and not any("segments" in m for m in ws.sent):
-            time.sleep(0.1)
-        client.exit = True
+        assert stand_in.ServeClientBase.done.wait(120)
         client.trans_thread.join(timeout=30)
-        segs = [m for m in ws.sent if "segments" in m]
-        assert segs, ws.sent
-        s0 = segs[0]["segments"][0]
-        assert set(s0) >= {"start", "end", "text", "completed"} and segs[0]["uid"] == "u1"
+        assert not stand_in.ServeClientBase.mismatches, stand_in.ServeClientBase.mismatches
+        # what the plugin sent itself; the segments message is the base's (checked above as send_transcription_to_client)
+        assert ws.sent == [m for m in rec["sent"] if "segments" not in m] and ws.sent[0]["message"] == "SERVER_READY"
+        segs = [m for m in rec["sent"] if "segments" in m]
+        assert segs and set(segs[0]["segments"][0]) >= {"start", "end", "text", "completed"} and segs[0]["uid"] == "u1"
     finally:
         BatchRequest.kwargs = orig_kwargs
-        ServeClientB200.shutdown()
-        ServeClientB200.MODEL_FACTORY = None
+        backend.ServeClientB200.shutdown()
+        backend.ServeClientB200.MODEL_FACTORY = None
+        for n, m in saved.items():
+            if m is None:
+                sys.modules.pop(n, None)
+            else:
+                sys.modules[n] = m
+        importlib.reload(backend)
 
 
 GLOO_WORKER = r"""
@@ -399,23 +392,52 @@ def test_bench_reference_arm_prints_the_contract_line():
     assert line["cpu_baseline"]["kind"] == "port" and line["cpu_baseline"]["cores"] >= 1 and "stand-in" in line["cpu_baseline"]["sample"]
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/whisper_live"), reason="reference tree only exists in the build container")
 def test_reference_batcher_runs_unmodified_on_the_b200_transcriber():
-    """SURVEY.md section 8(b): the reference's own BatchInferenceWorker (batch_inference.py:193-438), imported from the
-    reference tree, driven once over B200WhisperModel and once over the reference's WhisperModel (same CPU oracle engine
-    underneath) -- every request completes without error and the two runs agree segment for segment (tokens, times,
-    avg_logprob, no_speech_prob, temperature, language), for the batched path and the batch-of-one path."""
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    out = subprocess.run([sys.executable, os.path.join(root, "tests", "golden", "run_reference_batcher.py")], capture_output=True,
-                         text=True, timeout=600, cwd=root)
-    assert out.returncode == 0, out.stderr[-3000:]
-    res = json.loads(out.stdout.strip().splitlines()[-1])
-    assert set(res) == {"micro.en", "micro"}
-    for name, v in res.items():
-        mine, theirs = v["over_b200_model"], v["over_reference_model"]
-        assert len(mine) == 4 and all(r["error"] is None and r["done"] for r in mine), (name, mine)
-        assert all(r["segments"] for r in mine) and all(r["segment_type"] == "Segment" for r in mine)
-        assert mine == theirs, name
+    """SURVEY.md section 8(b): the reference's own BatchInferenceWorker (batch_inference.py:193-438) over the reference's
+    WhisperModel, recorded by tests/golden/run_reference_batcher.py for the batched path and the batch-of-one path: every
+    attribute it read and every call the transcriber answered (encode, get_prompt, _split_segments_by_timestamps,
+    transcribe) is replayed on B200WhisperModel over the same CPU oracle engine and must get the same answer -- so the
+    batcher driving B200WhisperModel agrees with the reference segment for segment (tokens, times, avg_logprob,
+    no_speech_prob, temperature, language)."""
+    from oracle import mel as omel
+    from oracle.engine import OracleWhisper
+    from oracle.mel import OracleFeatureExtractor
+    from tests.golden import run_reference_batcher as R
+    from whisperlive_b200.config import dims_for
+    from whisperlive_b200.tokenizer import Tokenizer, build_synthetic_tokenizer
+    from whisperlive_b200.transcriber import B200WhisperModel
+    from whisperlive_b200.weights import random_init
+    torch.set_num_threads(8)
+    gold = json.load(open(os.path.join(ROOT, "tests", "golden", "reference_batcher_calls.json")))
+    assert set(gold) == set(R.MODELS)
+    for name, log in gold.items():
+        dims = dims_for(name)
+        mine = B200WhisperModel(name, engine=OracleWhisper(random_init(dims, seed=0), dims),
+                                hf_tokenizer=build_synthetic_tokenizer(dims.vocab), feature_extractor=OracleFeatureExtractor(dims.n_mels))
+        waves = R.audios()
+
+        def tok(key):
+            return Tokenizer(mine.hf_tokenizer, key[0], task=key[1], language=key[2])
+        calls = [e.get("call") for e in log]
+        assert {"encode", "get_prompt", "_split_segments_by_timestamps", "transcribe"} <= set(calls), calls
+        for e in log:
+            if "attr" in e:
+                assert getattr(mine, e["attr"]) == e["value"], (name, e)
+            elif e["call"] == "encode":
+                feats = np.stack([omel.pad_or_trim(mine.feature_extractor(waves[i])) for i in e["audios"]])
+                np.testing.assert_allclose(R.encoder_sample(mine.encode(feats)), e["sample"], atol=1e-4, rtol=0)
+            elif e["call"] == "get_prompt":
+                assert list(mine.get_prompt(tok(e["tokenizer"]), **e["kwargs"])) == e["result"], (name, e)
+            elif e["call"] == "_split_segments_by_timestamps":
+                got = R.split_result(mine._split_segments_by_timestamps(tokenizer=tok(e["tokenizer"]), **e["kwargs"]))
+                assert got == e["result"], (name, got, e)
+            else:
+                segs, info = mine.transcribe(waves[e["audio"]], **e["kwargs"])
+                got, ref = R.result_row(None if segs is None else list(segs), info), e["result"]
+                assert ref["segments"] and got["segment_type"] == ref["segment_type"] == "Segment"
+                assert [s["tokens"] for s in got["segments"]] == [s["tokens"] for s in ref["segments"]], name
+                assert got["segments"] == pytest.approx(ref["segments"], abs=2e-6) and got["language"] == ref["language"]
+                assert got["duration"] == pytest.approx(ref["duration"])
 
 
 def test_bench_reference_arm_under_torchrun_two_ranks():
